@@ -15,8 +15,10 @@ line also carries a `strong` object (2^27 chains IN TOTAL, as configs[2] words i
 
   python bench.py [--gpus N --steps K --warmup W]                  # our arm (one process per GPU under torchrun)
   python bench.py --impl reference [...]                           # the CPU restatement of the reference path
+  python bench.py --dump-outputs DIR [...]                         # + the timed run's outputs as DIR/*.npy
 
-Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
+Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.  The inputs are seeded, so two builds
+run with the same arguments can be compared output for output through --dump-outputs (see dump_outputs).
 """
 from __future__ import annotations
 
@@ -62,7 +64,12 @@ def parse():
                          "else the largest power of two that does; cpu_baseline leg: 2^20)")
     ap.add_argument("--ref-seconds", type=float, default=120.0, help="time budget of the --impl reference run")
     ap.add_argument("--cpu-seconds", type=float, default=15.0, help="time budget of the cpu_baseline leg")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what they computed to DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -275,6 +282,27 @@ def launch_plan(K, g_max):
     return [min(g, K - s) for s in range(0, K, g)]
 
 
+DUMP_SAMPLE_CHAINS = 1 << 20          # 2 per-chain arrays x 8 B x 2^20 = 16 MiB: the whole dump stays under 64 MB
+
+
+def dump_outputs(out_dir, eng, records):
+    """Writes what the timed store intervals handed their caller, as float64 arrays in out_dir:
+      records.npy            [K][3] the callback record of every timed store interval (Σe, Σ acc/tot, chain count),
+                             summed over the ranks
+      x.npy, accepted.npy    position and accepted-move count after the last timed interval of a fixed sample of this
+                             rank's chains: DUMP_SAMPLE_CHAINS chain indices drawn with numpy's default_rng(0) without
+                             replacement, in ascending order (every chain when there are fewer).
+    The energies are not written: the engine derives them from the positions."""
+    os.makedirs(out_dir, exist_ok=True)
+    x = eng.get_state()
+    acc = eng.chain_counters()[0][0]
+    n = x.size
+    idx = np.arange(n) if n <= DUMP_SAMPLE_CHAINS else \
+        np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE_CHAINS, replace=False))
+    for name, a in (("records", records), ("x", x[idx]), ("accepted", acc[idx])):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+
 # ---------------------------------------------------------------------------------------------------------
 # our arm
 # ---------------------------------------------------------------------------------------------------------
@@ -376,6 +404,8 @@ def run_ours(args):
         fp64_peak = eng.measure_fp64_peak()
     main = timed_run(eng, m_local, K, W, True)
     rec = main["records"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, rec)           # before the e2e leg moves the chains on
     energy = float(rec[-1, 0] / rec[-1, 2])
     value = m_local * world * S * K / (main["ms"] * 1e-3)
 

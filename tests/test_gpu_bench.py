@@ -4,6 +4,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 pytestmark = pytest.mark.gpu
@@ -49,3 +50,23 @@ def test_bench_line_contract(series):
     assert p["x_bits_checksum_equals_1gpu"] in (True, None)
     c = d["cpu_baseline"]
     assert c["kind"] == "port" and c["cores"] >= 1 and c["value"] > 0 and c["unit"] == d["unit"] and c["sample"]
+
+
+def test_bench_dump_outputs_are_reproducible(tmp_path):
+    """--dump-outputs writes the timed run's outputs (one record per timed step, a 2^20-chain sample of the final
+    state) in float64, under 64 MB; the inputs are seeded, so a second run with the same arguments writes the same."""
+    names = ["accepted.npy", "records.npy", "x.npy"]
+    dumps = []
+    for run in ("a", "b"):
+        d = _run("--no-e2e", "--no-strong", "--no-parity", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / run))
+        assert sorted(os.listdir(tmp_path / run)) == names
+        assert sum(os.path.getsize(tmp_path / run / n) for n in names) <= 64 << 20
+        dumps.append({n: np.load(tmp_path / run / n) for n in names})
+        rec = dumps[-1]["records.npy"]
+        assert rec.shape == (25, 3) and np.all(rec[:, 2] == 1 << 22)           # one record per step of --steps 25
+        assert rec[-1, 0] / rec[-1, 2] == d["mean_energy"]
+    for n in names:
+        assert dumps[0][n].dtype == np.float64 and np.array_equal(dumps[0][n], dumps[1][n]), n
+    x, acc = dumps[0]["x.npy"], dumps[0]["accepted.npy"]
+    assert x.shape == acc.shape == (1 << 20,) and np.all(np.isfinite(x))
+    assert np.all((acc >= 0) & (acc <= 10 * (3 + 25)))         # 3 warm-up + 25 timed intervals of 10 steps
