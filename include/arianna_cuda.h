@@ -140,6 +140,27 @@ ARIANNA_API int32_t arianna_copy_wait(arianna_handle *h);
 ARIANNA_API int32_t arianna_set_beta(arianna_handle *h, double beta);
 ARIANNA_API int32_t arianna_set_betas(arianna_handle *h, const double *betas); /* per-chain β, [n_chains] host */
 
+/* Replica exchange (parallel tempering) across per-chain β ladders.  A ladder is L consecutive chains by GLOBAL index
+ * (2 <= L <= ARIANNA_MAX_LADDER); global chain g is rung g % L of ladder g / L.
+ * arianna_set_ladder writes per-chain β = betas[g % L] ([L] host), with the same effect as arianna_set_betas; the shard
+ * must hold whole ladders (chain_offset % L == 0 and n_chains % L == 0, ARIANNA_ERR_INVALID otherwise).  Calling it
+ * with another L resets the round index and the swap counters; later arianna_set_beta(s) calls are allowed (the
+ * exchange always reads the per-chain β).
+ * arianna_replica_exchange runs ONE round R (per handle, from 0): rungs (r, r + 1) with r ≡ R (mod 2) of every local
+ * ladder swap their positions x iff min(1, exp(Δ)) > u, Δ = (β_g − β_{g+1})·(e_g − e_{g+1}), e = potential(x) in exact
+ * binary64, u = (A >> 11)·2^-53 from the Philox stream tag 4 (sid = seed + g, p = R, sub 0), strict >, NaN rejects.  β,
+ * the Move counters and the chain's Metropolis stream stay with the slot (the temperature).  Asynchronous.
+ * arianna_exchange_counters: accepted swaps per rung pair [L − 1] (local shard) and the number of rounds; pair k was
+ * attempted n_ladders_local × #{R' < rounds : R' ≡ k (mod 2)} times.
+ * arianna_ladder_sums: the callback record restricted to each rung, [L][2 + n_moves] = (Σ e, Σ_c acc_ck/tot_ck per
+ * move, chain count) over the local shard, in a fixed reduction order; multi-GPU hosts sum them across ranks.
+ * Float64 ensembles with the native Philox stream (ARIANNA_ERR_UNSUPPORTED otherwise). */
+#define ARIANNA_MAX_LADDER 256
+ARIANNA_API int32_t arianna_set_ladder(arianna_handle *h, int32_t L, const double *betas);
+ARIANNA_API int32_t arianna_replica_exchange(arianna_handle *h);
+ARIANNA_API int32_t arianna_exchange_counters(arianna_handle *h, int64_t *accepted, int64_t *rounds);
+ARIANNA_API int32_t arianna_ladder_sums(arianna_handle *h, double *sums);
+
 /* Policy parameters θ = (σ) of move `move_id` (0-based): the shared `parameters` array every chain's Move
  * aliases (metropolis.jl:253-260), mutated in place by learning_step! (learning.jl:33).  P must be 1.
  * log_norm (optional, may be NULL) lets the host pass its own binary64 value of log(2π·σ²)/2

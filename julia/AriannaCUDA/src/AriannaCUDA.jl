@@ -18,7 +18,7 @@ using Libdl
 using Random
 
 export CudaEnsemble, callback_acceptance_cuda, flush!, device_positions, nccl_unique_id, comm_init!, plan!, run_host_job!,
-       device_update!
+       device_update!, set_ladder!, replica_exchange!, exchange_counters, ladder_sums
 
 const MAX_MOVES = 16
 const libarianna = Ref{String}(get(ENV, "ARIANNA_CUDA_LIB", "libarianna_cuda.so"))
@@ -322,6 +322,48 @@ function Arianna.store_trajectory(io, ens::CudaEnsemble, t::Int, ::Arianna.DAT)
     write(io, Int64(t))
     write(io, device_positions(ens))
     return nothing
+end
+
+# --- replica exchange (parallel tempering) across per-chain β ladders -----------------------------------------
+# Every L = length(betas) consecutive chains (global index) form one ladder, chain g at β = betas[g % L + 1]; the shard
+# (chain_offset, M) must hold whole ladders.  A `ReplicaExchange <: AriannaAlgorithm` whose make_step! calls
+# replica_exchange! sits next to Metropolis in algorithm_list.
+"""
+    set_ladder!(ens, betas)      per-chain β from a ladder of L = length(betas) rungs (arianna_set_ladder)
+    replica_exchange!(ens)       one exchange round, even / odd rung pairs alternating (arianna_replica_exchange)
+    exchange_counters(ens)       (accepted[L-1], attempted[L-1], rounds) of the local shard
+    ladder_sums(ens)             per-rung callback sums, L × (2 + n_moves): (Σe, Σ acc/tot per move, count)
+"""
+function set_ladder!(ens::CudaEnsemble, betas::Vector{Float64})
+    check(ens.handle, ccall((:arianna_set_ladder, libarianna[]), Int32, (Ptr{Cvoid}, Int32, Ptr{Float64}),
+                            ens.handle, length(betas), betas))
+    return nothing
+end
+
+function replica_exchange!(ens::CudaEnsemble)
+    flush!(ens)
+    check(ens.handle, ccall((:arianna_replica_exchange, libarianna[]), Int32, (Ptr{Cvoid},), ens.handle))
+    ens.cache_t = -1                              # the swap changed the energies behind the cached record
+    empty!(ens.series)
+    return nothing
+end
+
+function exchange_counters(ens::CudaEnsemble, L::Int)
+    acc = Vector{Int64}(undef, L - 1)
+    rounds = Ref{Int64}(0)
+    check(ens.handle, ccall((:arianna_exchange_counters, libarianna[]), Int32, (Ptr{Cvoid}, Ptr{Int64}, Ref{Int64}),
+                            ens.handle, acc, rounds))
+    R = rounds[]
+    attempted = [(getfield(ens, :M) ÷ L) * (iseven(k - 1) ? (R + 1) ÷ 2 : R ÷ 2) for k in 1:L-1]
+    return acc, attempted, R
+end
+
+function ladder_sums(ens::CudaEnsemble, L::Int)
+    flush!(ens)
+    w = 2 + length(getfield(ens, :pool))
+    out = Matrix{Float64}(undef, w, L)            # column r = the record of rung r (C row-major [L][w])
+    check(ens.handle, ccall((:arianna_ladder_sums, libarianna[]), Int32, (Ptr{Cvoid}, Ptr{Float64}), ens.handle, out))
+    return permutedims(out)
 end
 
 # --- PGMC ----------------------------------------------------------------------------------------------------

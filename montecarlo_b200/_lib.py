@@ -8,6 +8,7 @@ import os
 from ._build import LIB_PATH
 
 MAX_MOVES = 16
+MAX_LADDER = 256
 
 OK, ERR_INVALID, ERR_CUDA, ERR_NOMEM, ERR_UNSUPPORTED, ERR_NO_DEVICE, ERR_NCCL = range(7)
 POT_HARMONIC, POT_QUARTIC, POT_DOUBLE_WELL = 0, 1, 2
@@ -79,6 +80,10 @@ SYMBOLS = {
     "arianna_host_free": (C.c_int32, [C.c_void_p]),
     "arianna_set_beta": (C.c_int32, [_H, C.c_double]),
     "arianna_set_betas": (C.c_int32, [_H, C.c_void_p]),
+    "arianna_set_ladder": (C.c_int32, [_H, C.c_int32, _D]),
+    "arianna_replica_exchange": (C.c_int32, [_H]),
+    "arianna_exchange_counters": (C.c_int32, [_H, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "arianna_ladder_sums": (C.c_int32, [_H, _D]),
     "arianna_set_params": (C.c_int32, [_H, C.c_int32, _D, C.c_int32, _D]),
     "arianna_get_params": (C.c_int32, [_H, C.c_int32, _D, C.c_int32]),
     "arianna_sweep": (C.c_int32, [_H, C.c_int64, C.c_uint32]),

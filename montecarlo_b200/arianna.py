@@ -38,6 +38,7 @@ __all__ = [
     "StandardGaussian", "ComponentArray", "Move", "Metropolis", "Simulation", "run", "build_schedule",
     "StoreCallbacks", "StoreTrajectories", "StoreLastFrames", "StoreParameters", "PrintTimeSteps",
     "callback_energy", "callback_acceptance", "mc_sweep", "DAT", "TXT", "shard_bounds",
+    "ReplicaExchange", "callback_ladder_energy", "callback_ladder_acceptance", "callback_exchange_acceptance",
 ]
 
 
@@ -444,6 +445,82 @@ def callback_energy(simulation) -> float:
 def callback_acceptance(simulation):
     """Per-move mean over chains of accepted_calls / total_calls (metropolis.jl:319-321); NaN at t = 0."""
     return [float(v) for v in simulation.chains._callbacks()[1]]
+
+
+class ReplicaExchange(AriannaAlgorithm):
+    """ReplicaExchange(chains; dependencies=(Metropolis,), ladder): parallel tempering across per-chain β ladders.
+    Every L = len(ladder) consecutive chains (by global index) form one ladder, chain g at β = ladder[g % L].  Each call
+    runs ONE exchange round on the device: round R proposes to swap the positions of rungs (r, r + 1) with
+    r ≡ R (mod 2) in every ladder and accepts with min(1, exp((β_r − β_{r+1})(e_r − e_{r+1}))).  β and the Move
+    counters stay with the rung (the temperature), only the configurations travel.  Every rank's shard must hold whole
+    ladders."""
+
+    def __init__(self, chains, *, dependencies=None, ladder=None, **extras):
+        if not dependencies or len(dependencies) != 1 or not isinstance(dependencies[0], Metropolis):
+            raise TypeError("ReplicaExchange: dependencies=(Metropolis,) is required")
+        if ladder is None:
+            raise TypeError("ReplicaExchange: ladder (the β of each rung) is required")
+        self.ladder = np.ascontiguousarray(ladder, dtype=np.float64)
+        L = self.ladder.size
+        if self.ladder.ndim != 1 or not 2 <= L <= 256:
+            raise ValueError("ReplicaExchange: the ladder must have 2 to 256 rungs")
+        if chains.offset % L or chains.n_local % L:
+            raise ValueError(f"ReplicaExchange: the shard of rank {chains.rank}, chains [{chains.offset}, "
+                             f"{chains.offset + chains.n_local}), does not hold whole ladders of {L} chains")
+        chains.engine.set_ladder(self.ladder)
+        chains.betas = np.tile(self.ladder, chains.n_total // L)
+        chains.β = chains.beta = float(self.ladder[0])
+
+    def make_step(self, simulation):
+        ch = simulation.chains
+        ch.flush()
+        ch.engine.replica_exchange()
+        ch._cb_cache = None            # the swap changed the energies behind every cached record
+        ch._series_cache = {}
+
+    def write_algorithm(self, io, scheduler):
+        calls = sum(1 for x in scheduler if 0 < x <= scheduler[-1])
+        io.write(f"\tReplicaExchange\n\t\tCalls: {calls}\n")
+        io.write(f"\t\tLadder: {self.ladder.size} rungs\n\t\tβ: {_jl(list(self.ladder))}\n")
+        io.write(f"\t\tRounds: {calls} (one per call, even and odd rung pairs alternating)\n")
+
+
+def _allreduce_host(v: np.ndarray) -> np.ndarray:
+    """allreduce_sums of a host vector; under NCCL the collective needs a device copy of it."""
+    dist = _dist()
+    dev = None
+    if dist is not None and dist.get_world_size() > 1 and dist.get_backend() == "nccl":
+        import torch
+        dev = torch.from_numpy(np.ascontiguousarray(v)).cuda()
+    return allreduce_sums(v, dev)
+
+
+def _ladder_sums(simulation) -> np.ndarray:
+    ch = simulation.chains
+    ch.flush()
+    s = ch.engine.ladder_sums()
+    return _allreduce_host(s.reshape(-1)).reshape(s.shape)
+
+
+def callback_ladder_energy(simulation):
+    """Mean energy of every rung of the β ladder (ReplicaExchange): [L] values, ensemble-wide."""
+    s = _ladder_sums(simulation)
+    return [float(v) for v in s[:, 0] / s[:, -1]]
+
+
+def callback_ladder_acceptance(simulation):
+    """callback_acceptance restricted to each rung: per rung, the per-move mean of accepted_calls / total_calls."""
+    s = _ladder_sums(simulation)
+    with np.errstate(all="ignore"):
+        return [[float(v) for v in row[1:-1] / row[-1]] for row in s]
+
+
+def callback_exchange_acceptance(simulation):
+    """Accepted / attempted swaps of every rung pair (r, r + 1) since the ladder was set; NaN before the first attempt."""
+    acc, att, _ = simulation.chains.engine.exchange_counters()
+    tot = _allreduce_host(np.concatenate([acc, att]).astype(np.float64))
+    with np.errstate(all="ignore"):
+        return [float(v) for v in tot[:acc.size] / tot[acc.size:]]
 
 
 def _jl(v) -> str:

@@ -17,6 +17,7 @@
 
 #include "../../include/arianna_cuda.h"
 #include "kernels.cuh"
+#include "kernels_exchange.cuh"
 
 using namespace arianna;
 
@@ -61,6 +62,7 @@ static const char *load(std::string &err)
 
 static_assert(ARIANNA_MAX_MOVES == kMaxMoves, "header / kernel pool size mismatch");
 static_assert(ARIANNA_MAX_SERIES == kMaxSeries, "header / kernel series size mismatch");
+static_assert(ARIANNA_MAX_LADDER == kMaxLadder, "header / kernel ladder size mismatch");
 static_assert(sizeof(arianna_gradient_data) == 5 * sizeof(double), "gradient record layout");
 
 struct arianna_handle {
@@ -129,6 +131,13 @@ struct arianna_handle {
     int64_t pgmc_samples = 0;       // estimator samples drawn per chain
     int64_t launches = 0;
     bool sums_valid = false;
+
+    int ladder_L = 0;                      // replica exchange: rungs per ladder (0 = no ladder set)
+    int64_t ex_rounds = 0;                 // exchange rounds done (the round index R of the next one)
+    unsigned long long *d_xacc = nullptr;  // [kMaxLadder] accepted swaps per rung pair
+    double *d_ladder = nullptr;            // [L] the β ladder
+    double *d_ladder_partials = nullptr;   // [grid][L][1 + n_moves] of ladder_reduce_kernel
+    double *d_ladder_sums = nullptr;       // [L][2 + n_moves]
     std::string err;
 };
 
@@ -512,6 +521,7 @@ int32_t arianna_destroy(arianna_handle *h)
     cudaFree(h->d_sums); cudaFree(h->d_gd); cudaFree(h->d_csum); cudaFree(h->d_scratch); cudaFree(h->d_tables);
     cudaFree(h->d_series); cudaFree(h->d_series_partials); cudaFree(h->d_cat_table);
     cudaFree(h->d_pgmc_partials); cudaFree(h->d_pgmc_ticket); cudaFree(h->d_theta);
+    cudaFree(h->d_xacc); cudaFree(h->d_ladder); cudaFree(h->d_ladder_partials); cudaFree(h->d_ladder_sums);
     if (h->coll_stream) cudaStreamSynchronize(h->coll_stream);
     if (h->comm) { nccl::g_api.CommDestroy(h->comm); h->comm = nullptr; }
     cudaFree(h->d_coll);
@@ -1496,6 +1506,118 @@ int32_t arianna_callbacks(arianna_handle *h, double *mean_energy, double *acc_pe
     if (mean_energy) *mean_energy = sums[0] / cnt;
     if (acc_per_move)
         for (int k = 0; k < nm; ++k) acc_per_move[k] = sums[1 + k] / cnt;
+    return ARIANNA_OK;
+}
+
+// ---- replica exchange (parallel tempering) across per-chain β ladders (csrc/kernels_exchange.cuh) -----------------
+static int32_t ladder_supported(arianna_handle *h, const char *who)
+{
+    if (h->f32 || h->cfg.rng_mode != ARIANNA_RNG_PHILOX)
+        return fail(h, ARIANNA_ERR_UNSUPPORTED,
+                    std::string(who) + ": replica exchange needs a Float64 ensemble with the native Philox stream");
+    return ARIANNA_OK;
+}
+
+int32_t arianna_set_ladder(arianna_handle *h, int32_t L, const double *betas)
+{
+    if (!h) return ARIANNA_ERR_INVALID;
+    if (int32_t rc = ladder_supported(h, "arianna_set_ladder")) return rc;
+    REQUIRE(h, L >= 2 && L <= ARIANNA_MAX_LADDER, "arianna_set_ladder: L must be in 2..ARIANNA_MAX_LADDER");
+    REQUIRE(h, betas != nullptr, "arianna_set_ladder: betas is NULL");
+    REQUIRE(h, h->cfg.chain_offset % L == 0 && h->M % L == 0,
+            "arianna_set_ladder: the shard must hold whole ladders (chain_offset and n_chains multiples of L)");
+    DeviceGuard guard(h->device);
+    const int nm = h->pool.n_moves;
+    if (L != h->ladder_L) {             // another ladder shape: new buffers, fresh round index and counters
+        CU_TRY(h, cudaStreamSynchronize(h->stream));
+        cudaFree(h->d_ladder); cudaFree(h->d_ladder_partials); cudaFree(h->d_ladder_sums);
+        h->d_ladder = h->d_ladder_partials = h->d_ladder_sums = nullptr;
+        h->ladder_L = 0;
+        if (!h->d_xacc) CU_TRY(h, cudaMalloc(&h->d_xacc, sizeof(unsigned long long) * kMaxLadder));
+        CU_TRY(h, cudaMalloc(&h->d_ladder, sizeof(double) * L));
+        CU_TRY(h, cudaMalloc(&h->d_ladder_partials, sizeof(double) * (size_t)h->grid * L * (1 + nm)));
+        CU_TRY(h, cudaMalloc(&h->d_ladder_sums, sizeof(double) * (size_t)L * (2 + nm)));
+        CU_TRY(h, cudaMemsetAsync(h->d_xacc, 0, sizeof(unsigned long long) * kMaxLadder, h->stream));
+        h->ex_rounds = 0;
+    }
+    if (!h->d_betas) CU_TRY(h, cudaMalloc(&h->d_betas, sizeof(double) * h->M));
+    CU_TRY(h, cudaMemcpyAsync(h->d_ladder, betas, sizeof(double) * L, cudaMemcpyHostToDevice, h->stream));
+    ladder_betas_kernel<<<h->grid, kBlock, 0, h->stream>>>(h->d_betas, h->d_ladder, L, h->M);
+    CU_TRY(h, cudaGetLastError());
+    ++h->launches;
+    CU_TRY(h, cudaStreamSynchronize(h->stream));     // `betas` is borrowed for the call only
+    h->ladder_L = L;
+    return ARIANNA_OK;
+}
+
+int32_t arianna_replica_exchange(arianna_handle *h)
+{
+    if (!h) return ARIANNA_ERR_INVALID;
+    if (int32_t rc = ladder_supported(h, "arianna_replica_exchange")) return rc;
+    REQUIRE(h, h->ladder_L >= 2, "arianna_replica_exchange: no ladder (call arianna_set_ladder first)");
+    DeviceGuard guard(h->device);
+    const int L = h->ladder_L;
+    ExchangeParams p{};
+    p.x = h->d_x;
+    p.betas = h->d_betas;
+    p.beta = h->cfg.beta;
+    p.n_ladders = h->M / L;
+    p.L = L;
+    p.pairs = (L - (int)(h->ex_rounds & 1)) / 2;
+    p.R = h->ex_rounds;
+    p.sid0 = (uint64_t)(h->cfg.seed + h->cfg.chain_offset);
+    p.tables = h->d_tables;
+    p.accepted = h->d_xacc;
+    if (p.pairs > 0) {
+        dispatch_pot(h->cfg.potential, [&](auto pot) -> int32_t {
+            exchange_kernel<decltype(pot)::value><<<h->grid, kBlock, 0, h->stream>>>(p);
+            return ARIANNA_OK;
+        });
+        CU_TRY(h, cudaGetLastError());
+        ++h->launches;
+        h->sums_valid = false;
+    }
+    ++h->ex_rounds;
+    return ARIANNA_OK;
+}
+
+int32_t arianna_exchange_counters(arianna_handle *h, int64_t *accepted, int64_t *rounds)
+{
+    if (!h) return ARIANNA_ERR_INVALID;
+    if (int32_t rc = ladder_supported(h, "arianna_exchange_counters")) return rc;
+    REQUIRE(h, h->ladder_L >= 2, "arianna_exchange_counters: no ladder (call arianna_set_ladder first)");
+    DeviceGuard guard(h->device);
+    if (accepted) {
+        unsigned long long a[kMaxLadder];
+        CU_TRY(h, cudaMemcpyAsync(a, h->d_xacc, sizeof(unsigned long long) * (h->ladder_L - 1), cudaMemcpyDeviceToHost,
+                                  h->stream));
+        CU_TRY(h, cudaStreamSynchronize(h->stream));
+        for (int k = 0; k < h->ladder_L - 1; ++k) accepted[k] = (int64_t)a[k];
+    }
+    if (rounds) *rounds = h->ex_rounds;
+    return ARIANNA_OK;
+}
+
+int32_t arianna_ladder_sums(arianna_handle *h, double *sums)
+{
+    if (!h) return ARIANNA_ERR_INVALID;
+    if (int32_t rc = ladder_supported(h, "arianna_ladder_sums")) return rc;
+    REQUIRE(h, h->ladder_L >= 2, "arianna_ladder_sums: no ladder (call arianna_set_ladder first)");
+    REQUIRE(h, sums != nullptr, "arianna_ladder_sums: sums is NULL");
+    DeviceGuard guard(h->device);
+    const int L = h->ladder_L, nm = h->pool.n_moves;
+    LadderReduceParams p{h->d_x, h->d_acc, h->d_tot, h->M, h->M, h->steps_done, nm, h->cfg.potential, L,
+                         h->d_ladder_partials};
+    if (nm == 1) ladder_reduce_kernel<1><<<h->grid, kBlock, 0, h->stream>>>(p);
+    else ladder_reduce_kernel<kMaxMoves><<<h->grid, kBlock, 0, h->stream>>>(p);
+    CU_TRY(h, cudaGetLastError());
+    ++h->launches;
+    ladder_fold_kernel<<<L, kBlock, 0, h->stream>>>(h->d_ladder_partials, h->grid, L, nm, (double)(h->M / L),
+                                                    h->d_ladder_sums);
+    CU_TRY(h, cudaGetLastError());
+    ++h->launches;
+    CU_TRY(h, cudaMemcpyAsync(sums, h->d_ladder_sums, sizeof(double) * L * (2 + nm), cudaMemcpyDeviceToHost, h->stream));
+    CU_TRY(h, cudaStreamSynchronize(h->stream));
     return ARIANNA_OK;
 }
 

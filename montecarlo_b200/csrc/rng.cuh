@@ -16,7 +16,7 @@ constexpr uint32_t kPhiloxW0 = 0x9E3779B9u;
 constexpr uint32_t kPhiloxW1 = 0xBB67AE85u;
 constexpr uint32_t kKey1 = 0x41524941u;  // 'ARIA'
 
-enum : uint32_t { kTagInit = 0, kTagMetropolis = 1, kTagEstimator = 2 };
+enum : uint32_t { kTagInit = 0, kTagMetropolis = 1, kTagEstimator = 2, kTagExchange = 4 };
 
 struct U64Pair {
     uint32_t a_lo, a_hi, b_lo, b_hi;  // A = out[0] | out[1] << 32,  B = out[2] | out[3] << 32

@@ -99,6 +99,7 @@ class CudaEnsemble:
         self.seed = int(seed)
         self.beta = float(beta)
         self.rng, self.arith, self.potential = rng, arith, potential
+        self.ladder = None
 
     # -- lifecycle ----------------------------------------------------------------------------------------
     def close(self):
@@ -173,6 +174,40 @@ class CudaEnsemble:
         if b.shape != (self.n_chains,):
             raise ValueError(f"betas must have shape ({self.n_chains},)")
         self._ck(self._lib.arianna_set_betas(self._h, _ptr(b)))
+
+    # -- replica exchange across β ladders ----------------------------------------------------------------
+    def set_ladder(self, betas):
+        """β ladder of L = len(betas) rungs: chain g (global) gets betas[g % L] (arianna_set_ladder).  The shard must
+        hold whole ladders."""
+        b = np.ascontiguousarray(betas, dtype=np.float64)
+        if b.ndim != 1:
+            raise ValueError("betas must be a 1-d ladder")
+        self._ck(self._lib.arianna_set_ladder(self._h, int(b.size), b.ctypes.data_as(C.POINTER(C.c_double))))
+        self.ladder = b.copy()
+
+    def _rungs(self) -> int:
+        # without a ladder the library refuses the call; the buffer only has to be large enough until it does
+        return self.ladder.size if self.ladder is not None else L.MAX_LADDER
+
+    def replica_exchange(self):
+        """One exchange round between neighbouring rungs, even/odd pairs alternating (asynchronous)."""
+        self._ck(self._lib.arianna_replica_exchange(self._h))
+
+    def exchange_counters(self):
+        """(accepted[L-1], attempted[L-1], rounds) of the local shard; pair k is attempted in rounds R ≡ k (mod 2)."""
+        n = self._rungs()
+        acc = (C.c_int64 * (n - 1))()
+        rounds = C.c_int64()
+        self._ck(self._lib.arianna_exchange_counters(self._h, acc, C.byref(rounds)))
+        R = rounds.value
+        per_round = np.array([(R + 1) // 2 if k % 2 == 0 else R // 2 for k in range(n - 1)], dtype=np.int64)
+        return np.array(acc[:], dtype=np.int64), (self.n_chains // n) * per_round, R
+
+    def ladder_sums(self):
+        """Per-rung callback records [L][2 + n_moves] = (Σe, Σ acc/tot per move, count) over the local shard."""
+        out = np.empty((self._rungs(), 2 + self.n_moves), dtype=np.float64)
+        self._ck(self._lib.arianna_ladder_sums(self._h, out.ctypes.data_as(C.POINTER(C.c_double))))
+        return out
 
     # -- policy parameters --------------------------------------------------------------------------------
     def set_params(self, move_id: int, sigma: float, log_norm: Optional[float] = None):
