@@ -26,6 +26,9 @@ def _ladder(rng, L):
 @pytest.mark.parametrize("M,L,pot,sigma,weight", [
     (1 << 16, 8, "harmonic", [0.3], [1.0]),
     (5 << 13, 5, "double_well", [0.3, 0.05], [0.5, 0.5]),
+    (6 << 12, 6, "quartic", [0.3], [1.0]),
+    (1 << 14, 2, "double_well", [0.4], [1.0]),                          # one rung pair
+    (120 << 8, 256, "harmonic", [0.3, 0.1, 0.05], [0.5, 0.25, 0.25]),   # kMaxLadder rungs: 255 swap counters
 ])
 def test_parity_with_the_oracle(M, L, pot, sigma, weight):
     """EXACT: the device replays the native stream's draws (draws_philox) and runs its own exchange rounds; the oracle
@@ -46,6 +49,9 @@ def test_parity_with_the_oracle(M, L, pot, sigma, weight):
         xacc += XO.exchange(ref, L, seed, R, 0, betas=betas)
         done += K
     assert 0 < xacc.sum() < (M // L) * (L - 1) * len(SCHEDULE) // 2
+    assert 0.05 < ref.acc.sum() / ref.tot.sum() < 0.95                # a wrong potential or β would show
+    if pot == "double_well":
+        assert 0 < np.count_nonzero(ref.x < 0) < M
     ref_sums = XO.ladder_sums(ref, L)
     for arith in ("exact", "fast"):
         with mb.CudaEnsemble(M, 1.0, sigma, weight, seed=seed, potential=pot, arith=arith) as eng:
