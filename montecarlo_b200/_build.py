@@ -9,7 +9,7 @@ import subprocess
 _HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_HERE, "csrc")
 INCLUDE = os.path.join(os.path.dirname(_HERE), "include")
-LIB_PATH = os.environ.get("ARIANNA_LIB") or os.path.join(_HERE, "libarianna_cuda.so")
+LIB_PATH = os.path.join(_HERE, "libarianna_cuda.so")
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
@@ -31,22 +31,21 @@ def is_stale() -> bool:
     return any(os.path.getmtime(s) > t for s in _sources())
 
 
-def build_library(force: bool = False, verbose: bool = False, defines=(), out: str = None) -> str:
-    """Compile csrc/arianna_cuda.cu -> montecarlo_b200/libarianna_cuda.so.  Needs nvcc; no GPU required.
-    `defines` / `out` build A/B variants of the tuning knobs (scripts/ab_variants.sh)."""
-    if out is None and not force and not is_stale():
+def build_library(force: bool = False, verbose: bool = False) -> str:
+    """Compile csrc/arianna_cuda.cu -> montecarlo_b200/libarianna_cuda.so.  Needs nvcc; no GPU required."""
+    if not force and not is_stale():
         return LIB_PATH
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
     if not os.path.exists(nvcc):
         raise RuntimeError("nvcc not found: cannot build libarianna_cuda.so (there is no CPU fallback)")
-    cmd = [nvcc] + NVCC_FLAGS + [f"-D{d}" for d in defines] + (["-Xptxas", "-v"] if verbose else []) + [
-        "-o", out or LIB_PATH, os.path.join(CSRC, "arianna_cuda.cu")]
+    cmd = [nvcc] + NVCC_FLAGS + (["-Xptxas", "-v"] if verbose else []) + [
+        "-o", LIB_PATH, os.path.join(CSRC, "arianna_cuda.cu")]
     res = subprocess.run(cmd, capture_output=True, text=True)
     if res.returncode != 0:
         raise RuntimeError("nvcc failed:\n" + res.stdout + res.stderr)
     if verbose:
         print(res.stderr)
-    return out or LIB_PATH
+    return LIB_PATH
 
 
 if __name__ == "__main__":

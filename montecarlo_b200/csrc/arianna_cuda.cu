@@ -309,7 +309,6 @@ int32_t ensure_series_partials(arianna_handle *h, size_t n_doubles);
 // 16 waves the hardware CTA scheduler staggers the phases and balances the tail; measured on M = 2^27, K = 10:
 // 1 / 2 / 4 / 8 / 16 / 32 / 64 / 256 waves -> 5.57 / 5.28 / 5.15 / 5.09 / 5.06 / 5.07 / 5.11 / 5.36 ms.
 constexpr int kGridWaves = 16;
-constexpr int kMaxGridWaves = 32;
 template <typename K>
 int wave_grid(const arianna_handle *h, K kernel, size_t smem, int64_t M)
 {
@@ -319,11 +318,11 @@ int wave_grid(const arianna_handle *h, K kernel, size_t smem, int64_t M)
         per_sm = 2;
     }
     if (per_sm > 8) per_sm = 8;
-    static const int env_waves = getenv("ARIANNA_GRID_WAVES") ? atoi(getenv("ARIANNA_GRID_WAVES")) : 0;
-    int waves = env_waves > 0 ? env_waves : kGridWaves;
-    if (waves > kMaxGridWaves) waves = kMaxGridWaves;
-    return grid_for(h, M, per_sm * waves);
+    return grid_for(h, M, per_sm * kGridWaves);
 }
+
+// the largest grid wave_grid() can return: what the per-CTA partial buffers are sized for
+int max_wave_grid(const arianna_handle *h) { return h->sm_count * 8 * kGridWaves; }
 
 int32_t ensure_series_partials(arianna_handle *h, size_t n_doubles)
 {
@@ -472,8 +471,7 @@ int32_t arianna_create(const arianna_config *cfg, arianna_handle **out)
         CU_CREATE(cudaStreamSynchronize(h->stream));
     }
     if (!h->f32) CU_CREATE(cudaMemsetAsync(h->d_x, 0, sizeof(double) * h->M, h->stream));
-    const int max_grid = h->sm_count * 8 * kMaxGridWaves;  // partials of the largest grid wave_grid() can return
-    CU_CREATE(cudaMalloc(&h->d_partials, sizeof(double) * (size_t)max_grid * kMaxOut));
+    CU_CREATE(cudaMalloc(&h->d_partials, sizeof(double) * (size_t)max_wave_grid(h) * kMaxOut));
     CU_CREATE(cudaMalloc(&h->d_ticket, sizeof(unsigned int)));
     CU_CREATE(cudaMemsetAsync(h->d_ticket, 0, sizeof(unsigned int), h->stream));
     CU_CREATE(cudaMalloc(&h->d_sums, sizeof(double) * kMaxOut));
@@ -831,9 +829,8 @@ static int32_t launch_multi(arianna_handle *h, int64_t off, int64_t m, int64_t t
     mp.K[n_int] = 0;
     mp.even = even ? 1 : 0;
     mp.pitch = h->M;
-    // two counter buffers (prefetch of the next chain's counters) when that still leaves ARIANNA_MULTI_MINB CTAs per SM
-    mp.dbuf = multi_smem_bytes(nm, n_int, mp.record, 1) + 1024 <= h->smem_per_sm / ARIANNA_MULTI_MINB ? 1 : 0;
-    if (const char *e = getenv("ARIANNA_MULTI_DBUF")) mp.dbuf = atoi(e) ? 1 : 0;
+    // two counter buffers (prefetch of the next chain's counters) when that still leaves kMultiMinBlocks CTAs per SM
+    mp.dbuf = multi_smem_bytes(nm, n_int, mp.record, 1) + 1024 <= h->smem_per_sm / kMultiMinBlocks ? 1 : 0;
     const size_t smem = multi_smem_bytes(nm, n_int, mp.record, mp.dbuf);
     int grid = 0;
     int32_t rc = dispatch_pot(h->cfg.potential, [&](auto pot) -> int32_t {
@@ -990,13 +987,14 @@ int32_t arianna_sweep(arianna_handle *h, int64_t K, uint32_t flags)
 // count: the reference's own small-M configurations) fuses up to ARIANNA_MAX_SERIES per launch.
 static int series_per_launch(const arianna_handle *h)
 {
-    const char *e = getenv("ARIANNA_SERIES_PER_LAUNCH");   // test / tuning override
+    // test hook (with ARIANNA_REPLAY_STAGE_BYTES): a small value forces the multi-launch splits the tests cover
+    const char *e = getenv("ARIANNA_SERIES_PER_LAUNCH");
     const int env = e ? atoi(e) : 0;
     if (env > 0) return env < kMaxSeries ? env : kMaxSeries;
     if (h->pool.n_moves > 1) {
         // multi-move pools: one warp-accumulator row of (1 + n_moves) doubles per interval and warp; as many intervals
-        // as keep ARIANNA_MULTI_MINB CTAs per SM, at most 32 (the per-CTA partials grow with it)
-        const long budget = (long)(h->smem_per_sm / ARIANNA_MULTI_MINB) - 1024 - (long)multi_smem_bytes(h->pool.n_moves, 0, 0, 1);
+        // as keep kMultiMinBlocks CTAs per SM, at most 32 (the per-CTA partials grow with it)
+        const long budget = (long)(h->smem_per_sm / kMultiMinBlocks) - 1024 - (long)multi_smem_bytes(h->pool.n_moves, 0, 0, 1);
         long n = budget / (long)(kWarpsPerBlock * (1 + h->pool.n_moves) * 8);
         if (n < 1) n = 1;
         if (n > 32) n = 32;
@@ -1009,7 +1007,7 @@ static int series_per_launch(const arianna_handle *h)
         stat = fa.sharedSizeBytes;
     else
         cudaGetLastError();
-    const long per_cta = (long)(h->smem_per_sm / ARIANNA_MINB) - 1024 - (long)stat - (long)sizeof(m64::MathTables) -
+    const long per_cta = (long)(h->smem_per_sm / kSweepMinBlocks) - 1024 - (long)stat - (long)sizeof(m64::MathTables) -
                          (long)(sizeof(unsigned long long) * kBlock);
     long n = per_cta / kSeriesBytesPerStore;
     if (n < 1) n = 1;
@@ -1119,13 +1117,9 @@ static int32_t series_prepare(arianna_handle *h, const char *who, int32_t n_stor
     // middle of a pipelined host job means cudaFree, i.e. a device-wide synchronisation that waits for every queued
     // upload (measured: the regular slices of a job started only after the whole ensemble had been uploaded).
     {
-        static const int env_waves = getenv("ARIANNA_GRID_WAVES") ? atoi(getenv("ARIANNA_GRID_WAVES")) : 0;
-        int waves = env_waves > 0 ? env_waves : kGridWaves;
-        if (waves > kMaxGridWaves) waves = kMaxGridWaves;
-        const size_t max_grid = (size_t)h->sm_count * 8 * waves;
         const int per_launch = series_per_launch(h);
         const size_t per_cta = h->pool.n_moves > 1 ? (size_t)per_launch * (1 + h->pool.n_moves) : (size_t)(per_launch + 1) * 2;
-        const int32_t rc = ensure_series_partials(h, max_grid * per_cta);
+        const int32_t rc = ensure_series_partials(h, (size_t)max_wave_grid(h) * per_cta);
         if (rc) return rc;
     }
     return ARIANNA_OK;
@@ -1368,8 +1362,7 @@ int32_t arianna_sweep_replay(arianna_handle *h, int64_t K, const double *u_cat, 
         // bulk-copy (TMA) path: cp.async.bulk needs 16-byte aligned rows, i.e. an even number of chains and 16-byte
         // aligned arrays; ragged shapes take the per-thread-load kernel (same arithmetic, same results)
         auto aligned16 = [](const void *q) { return (reinterpret_cast<uintptr_t>(q) & 15u) == 0; };
-        static const int env_tma = getenv("ARIANNA_REPLAY_TMA") ? atoi(getenv("ARIANNA_REPLAY_TMA")) : 1;
-        const bool tma = env_tma && (h->M % 2 == 0) && aligned16(dz) && aligned16(dua) && (!multi || aligned16(duc));
+        const bool tma = (h->M % 2 == 0) && aligned16(dz) && aligned16(dua) && (!multi || aligned16(duc));
         auto go_tma = [&](auto kernel) -> int32_t {
             const size_t dyn = replay_tma_smem_bytes(h->pool.n_moves);
             CU_TRY(h, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dyn));
@@ -1400,6 +1393,7 @@ int32_t arianna_sweep_replay(arianna_handle *h, int64_t K, const double *u_cat, 
         // stage host draws through a bounded device buffer, chunked over steps (<= 1 GiB per array)
         const size_t per_step = sizeof(double) * (size_t)h->M;
         size_t stage = size_t(1) << 30;
+        // test hook (with ARIANNA_SERIES_PER_LAUNCH): a small value forces the chunking the tests cover
         if (const char *env = getenv("ARIANNA_REPLAY_STAGE_BYTES")) stage = (size_t)strtoull(env, nullptr, 10);
         int64_t kc = (int64_t)(stage / per_step);
         if (kc < 1) kc = 1;

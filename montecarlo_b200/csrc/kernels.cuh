@@ -23,25 +23,12 @@
 
 namespace arianna {
 
-// Tuning knobs of the fused sweep (overridable for A/B builds, see scripts/ab_variants.sh):
-//   ARIANNA_MINB  resident CTAs per SM requested through __launch_bounds__ (register cap = 65536 / (256·MINB))
-//   ARIANNA_BLOCK threads per CTA (multiple of 32)
-//   ARIANNA_PGMC_MINB the same for the PGMC estimator kernel
-//   ARIANNA_PIPE  1 = software-pipeline the Box-Muller/Philox work of pair p+1 over the two steps of pair p
-#ifndef ARIANNA_MINB
-#define ARIANNA_MINB 4
-#endif
-#ifndef ARIANNA_PIPE
-#define ARIANNA_PIPE 0
-#endif
-#ifndef ARIANNA_PGMC_MINB
-#define ARIANNA_PGMC_MINB 3   // the estimator (a full FP64 exp per sample) prefers 80 registers x 3 CTAs: 4.20 vs 4.39 ms (C4)
-#endif
-
-#ifndef ARIANNA_BLOCK
-#define ARIANNA_BLOCK 256
-#endif
-constexpr int kBlock = ARIANNA_BLOCK;
+// Launch shape of the fused sweep: kBlock threads per CTA (a multiple of 32) and kSweepMinBlocks resident CTAs per SM
+// requested through __launch_bounds__, i.e. a cap of 65536 / (256·4) = 64 registers.  The measured optimum: 3, 5 or 6
+// CTAs per SM and a software pipeline of pair p+1 over pair p were all slower (DESIGN.md §4).
+constexpr int kBlock = 256;
+constexpr int kSweepMinBlocks = 4;
+constexpr int kPgmcMinBlocks = 3;   // the estimator (a full FP64 exp per sample) prefers 80 registers x 3 CTAs: 4.20 vs 4.39 ms (C4)
 constexpr int kMaxMoves = 16;
 constexpr int kMaxSeries = 64;              // store intervals one series launch can fuse (host picks <= this)
 constexpr int kSeriesBytesPerStore = kBlock * (8 + 4);   // shared memory per fused interval: Σe f64 + ΣΔacc u32 per thread
@@ -334,7 +321,7 @@ __device__ __forceinline__ void block_reduce_and_finish(const double *vals, int 
 // turns the partials into one [Σe, Σacc/t, count] record per store.  No host round trip and no second launch per
 // store: StoreCallbacks at every 10th step costs the same as one K = 10·n_series sweep.
 template <int POT, int ARITH, bool SERIES = false, bool BETAS = true>
-__global__ void __launch_bounds__(kBlock, ARIANNA_MINB) sweep_philox_kernel(const SweepParams p)
+__global__ void __launch_bounds__(kBlock, kSweepMinBlocks) sweep_philox_kernel(const SweepParams p)
 {
     // dynamic shared memory: [MathTables][kernel-specific arrays] -- ONE symbol, so one pinned base register serves
     // the math tables and the series accumulators alike
@@ -451,24 +438,8 @@ __global__ void __launch_bounds__(kBlock, ARIANNA_MINB) sweep_philox_kernel(cons
         const bool trail = ((tb - tfull) & 1u) != 0;
         uint64_t pr = (uint64_t)(ta >> 1);
         if (lead) { do_steps(gen_pair(pr), F_{}, T_{}); ++pr; }
-#if ARIANNA_PIPE
-        // Software pipeline: the draws of pair p+1 are generated while the serial accept chain of pair p runs, so
-        // every warp carries two independent dependency chains (the sweep is FP64-latency bound, not issue bound).
-        if (npairs > 0) {
-            PairDraws cur = gen_pair(pr);
-#pragma unroll 1
-            for (int i = 1; i < npairs; ++i) {
-                const PairDraws nxt = gen_pair(pr + (uint64_t)i);
-                do_steps(cur, T_{}, T_{});
-                cur = nxt;
-            }
-            do_steps(cur, T_{}, T_{});
-            pr += (uint64_t)npairs;
-        }
-#else
 #pragma unroll 1
         for (int i = 0; i < npairs; ++i, ++pr) do_steps(gen_pair(pr), T_{}, T_{});
-#endif
         if (trail) do_steps(gen_pair(pr), T_{}, F_{});
         };
         if constexpr (SERIES) {
@@ -925,7 +896,7 @@ __device__ __forceinline__ void pgmc_sample(double &x, double &e, double beta, d
 }
 
 template <int POT, int ARITH, bool REPLAY>
-__global__ void __launch_bounds__(kBlock, ARIANNA_PGMC_MINB) pgmc_kernel(const PgmcParams p)
+__global__ void __launch_bounds__(kBlock, kPgmcMinBlocks) pgmc_kernel(const PgmcParams p)
 {
     __shared__ m64::MathTables s_T;
     load_tables(&s_T, p.tables);

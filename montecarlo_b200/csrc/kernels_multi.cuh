@@ -24,9 +24,7 @@
 
 namespace arianna {
 
-#ifndef ARIANNA_MULTI_MINB
-#define ARIANNA_MULTI_MINB 4
-#endif
+constexpr int kMultiMinBlocks = 4;  // resident CTAs per SM; the host sizes shared memory (buffers, intervals) to keep them
 constexpr int kCatBuckets = 4096;   // top 12 bits of the 32-bit categorical word
 
 struct MultiParams {
@@ -87,7 +85,7 @@ __host__ __device__ constexpr size_t multi_smem_bytes(int n_moves, int n_int, in
 }
 
 template <int POT, int ARITH, bool BETAS>
-__global__ void __launch_bounds__(kBlock, ARIANNA_MULTI_MINB) sweep_multi_kernel(const MultiParams p)
+__global__ void __launch_bounds__(kBlock, kMultiMinBlocks) sweep_multi_kernel(const MultiParams p)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr uint32_t kTabBytes = (uint32_t)sizeof(m64::MathTables);
