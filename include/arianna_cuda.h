@@ -161,6 +161,31 @@ ARIANNA_API int32_t arianna_replica_exchange(arianna_handle *h);
 ARIANNA_API int32_t arianna_exchange_counters(arianna_handle *h, int64_t *accepted, int64_t *rounds);
 ARIANNA_API int32_t arianna_ladder_sums(arianna_handle *h, double *sums);
 
+/* Histograms and moments of the chains' current state, reduced on the device (StoreTrajectories + a host histogram
+ * without the download).  observable: ARIANNA_OBS_X the position, ARIANNA_OBS_E the energy potential(x) (Float64
+ * handles: exact binary64; Float32 handles: Float64(potential_f32(x)), i.e. what arianna_get_state_f32 returns, widened).
+ * Global chain g = chain_offset + c belongs to group g % n_groups (1 <= n_groups <= ARIANNA_MAX_LADDER; 1 = the whole
+ * ensemble, L = the rungs of a replica-exchange ladder); counts of any sharding sum to the one-handle counts.
+ * Bin rule (a formula, not edges): inv_w = n_bins / (hi − lo) in binary64, computed once by arianna_set_histogram;
+ * k = floor((v − lo)·inv_w) with the subtraction and the product rounded separately (no contraction).  NaN -> the nan
+ * cell, k < 0 -> underflow, k >= n_bins -> overflow (±inf land there), otherwise bin k.
+ * counts [n_groups][n_bins + 3] int64 = [n_bins regular][underflow][overflow][nan]; moments [n_groups][3] =
+ * (n, Σv, Σv²) over the finite v, binary64 sums in a fixed order (deterministic for a handle).
+ * arianna_set_histogram allocates and zeroes the accumulators (a second call replaces the binning);
+ * n_groups·(n_bins + 3) <= ARIANNA_MAX_HISTOGRAM_CELLS, n_bins >= 1, lo and hi finite, lo < hi, inv_w finite and > 0.
+ * arianna_histogram_accumulate adds one sample of every local chain (asynchronous; reads x only: no callback record,
+ * series record, counter, β, σ or step count changes).  arianna_histogram_read returns the local-shard accumulators
+ * and the number of accumulate calls (any pointer may be NULL; synchronises); multi-GPU hosts sum counts and moments
+ * across ranks.  arianna_histogram_reset zeroes counts, moments and the call count and keeps the binning.
+ * ARIANNA_ERR_INVALID for bad arguments and for accumulate / read / reset before arianna_set_histogram. */
+#define ARIANNA_MAX_HISTOGRAM_CELLS 16384
+enum arianna_observable { ARIANNA_OBS_X = 0, ARIANNA_OBS_E = 1 };
+ARIANNA_API int32_t arianna_set_histogram(arianna_handle *h, int32_t observable, double lo, double hi, int32_t n_bins,
+                                          int32_t n_groups);
+ARIANNA_API int32_t arianna_histogram_accumulate(arianna_handle *h);
+ARIANNA_API int32_t arianna_histogram_read(arianna_handle *h, int64_t *counts, double *moments, int64_t *n_samples);
+ARIANNA_API int32_t arianna_histogram_reset(arianna_handle *h);
+
 /* Policy parameters θ = (σ) of move `move_id` (0-based): the shared `parameters` array every chain's Move
  * aliases (metropolis.jl:253-260), mutated in place by learning_step! (learning.jl:33).  P must be 1.
  * log_norm (optional, may be NULL) lets the host pass its own binary64 value of log(2π·σ²)/2

@@ -18,7 +18,8 @@ using Libdl
 using Random
 
 export CudaEnsemble, callback_acceptance_cuda, flush!, device_positions, nccl_unique_id, comm_init!, plan!, run_host_job!,
-       device_update!, set_ladder!, replica_exchange!, exchange_counters, ladder_sums
+       device_update!, set_ladder!, replica_exchange!, exchange_counters, ladder_sums, set_histogram!,
+       accumulate_histogram!, histogram, reset_histogram!
 
 const MAX_MOVES = 16
 const libarianna = Ref{String}(get(ENV, "ARIANNA_CUDA_LIB", "libarianna_cuda.so"))
@@ -86,6 +87,7 @@ mutable struct CudaEnsemble{T<:AbstractFloat} <: AriannaSystem
     ahead::Int
     series::Dict{Int,Tuple{Float64,Vector{Float64}}}
     lookahead::Any
+    hist_shape::Tuple{Int,Int}  # (groups, bins + 3) of the on-device histogram, (0, 0) before set_histogram!
 end
 
 function CudaEnsemble(x0::Vector{Float64}, β::Float64, pool; seed::Int=1, potential::Symbol=:harmonic,
@@ -100,7 +102,7 @@ function CudaEnsemble(x0::Vector{Float64}, β::Float64, pool; seed::Int=1, poten
     h = Ref{Ptr{Cvoid}}(C_NULL)
     check(C_NULL, ccall((:arianna_create, libarianna[]), Int32, (Ref{AriannaConfig}, Ref{Ptr{Cvoid}}), cfg, h))
     ens = CudaEnsemble{Float64}(h[], length(x0), β, pool, 0, -1, NaN, fill(NaN, nm), 0,
-                                Dict{Int,Tuple{Float64,Vector{Float64}}}(), nothing)
+                                Dict{Int,Tuple{Float64,Vector{Float64}}}(), nothing, (0, 0))
     check(ens.handle, ccall((:arianna_set_state, libarianna[]), Int32, (Ptr{Cvoid}, Ptr{Float64}), ens.handle, x0))
     if rng == :xoshiro
         # the reference's own generators, rngs = [Xoshiro(seed + c - 1) for c in 1:M] (metropolis.jl:262-263), run on the
@@ -365,6 +367,44 @@ function ladder_sums(ens::CudaEnsemble, L::Int)
     check(ens.handle, ccall((:arianna_ladder_sums, libarianna[]), Int32, (Ptr{Cvoid}, Ptr{Float64}), ens.handle, out))
     return permutedims(out)
 end
+
+# --- on-device histograms and moments of x or e ----------------------------------------------------------------
+"""
+    set_histogram!(ens, observable, lo, hi, bins; groups=1)   observable :x (position) or :e (energy) (arianna_set_histogram)
+    accumulate_histogram!(ens)     one sample of every chain's current state, after the pending steps (asynchronous)
+    histogram(ens) -> (counts::Matrix{Int64}, moments::Matrix{Float64}, n_samples)
+    reset_histogram!(ens)          zero the accumulators, keep the binning
+
+Chain g (global, 0-based) is in group g % groups.  Bin of v: floor((v - lo) * inv_w), inv_w = bins / (hi - lo) in
+Float64, the subtraction and the product rounded separately.  counts is groups × (bins + 3): the bins, underflow,
+overflow, NaN; moments is groups × 3: (n, Σv, Σv²) over the finite v; both for the local shard (sum them across ranks).
+"""
+function set_histogram!(ens::CudaEnsemble, observable::Symbol, lo::Float64, hi::Float64, bins::Int; groups::Int=1)
+    observable in (:x, :e) || throw(ArgumentError("observable must be :x or :e"))
+    check(ens.handle, ccall((:arianna_set_histogram, libarianna[]), Int32, (Ptr{Cvoid}, Int32, Float64, Float64, Int32, Int32),
+                            ens.handle, observable === :x ? 0 : 1, lo, hi, bins, groups))
+    ens.hist_shape = (groups, bins + 3)
+    return nothing
+end
+
+function accumulate_histogram!(ens::CudaEnsemble)
+    flush!(ens)
+    check(ens.handle, ccall((:arianna_histogram_accumulate, libarianna[]), Int32, (Ptr{Cvoid},), ens.handle))
+    return nothing
+end
+
+function histogram(ens::CudaEnsemble)
+    G, cells = getfield(ens, :hist_shape)
+    counts = Matrix{Int64}(undef, cells, G)       # column g = group g (C row-major [G][bins + 3])
+    moments = Matrix{Float64}(undef, 3, G)
+    n = Ref{Int64}(0)
+    check(ens.handle, ccall((:arianna_histogram_read, libarianna[]), Int32, (Ptr{Cvoid}, Ptr{Int64}, Ptr{Float64}, Ref{Int64}),
+                            ens.handle, counts, moments, n))
+    return permutedims(counts), permutedims(moments), n[]
+end
+
+reset_histogram!(ens::CudaEnsemble) =
+    check(ens.handle, ccall((:arianna_histogram_reset, libarianna[]), Int32, (Ptr{Cvoid},), ens.handle))
 
 # --- PGMC ----------------------------------------------------------------------------------------------------
 # make_step!(sim, ::PolicyGradientEstimator) (estimator.jl:111-134) for a simulation whose chains are device-resident:

@@ -9,17 +9,20 @@ from ._build import LIB_PATH
 
 MAX_MOVES = 16
 MAX_LADDER = 256
+MAX_HISTOGRAM_CELLS = 16384
 
 OK, ERR_INVALID, ERR_CUDA, ERR_NOMEM, ERR_UNSUPPORTED, ERR_NO_DEVICE, ERR_NCCL = range(7)
 POT_HARMONIC, POT_QUARTIC, POT_DOUBLE_WELL = 0, 1, 2
 RNG_PHILOX, RNG_XOSHIRO = 0, 1
 ARITH_EXACT, ARITH_FAST = 0, 1
 SWEEP_REDUCE = 1
+OBS_X, OBS_E = 0, 1
 
 POTENTIALS = {"harmonic": POT_HARMONIC, "quartic": POT_QUARTIC, "double_well": POT_DOUBLE_WELL}
 RNG_MODES = {"philox": RNG_PHILOX, "xoshiro": RNG_XOSHIRO}
 ARITH_MODES = {"exact": ARITH_EXACT, "fast": ARITH_FAST}
 DTYPES = {"f64": 0, "f32": 1}
+OBSERVABLES = {"x": OBS_X, "e": OBS_E}
 
 
 class Config(C.Structure):
@@ -84,6 +87,10 @@ SYMBOLS = {
     "arianna_replica_exchange": (C.c_int32, [_H]),
     "arianna_exchange_counters": (C.c_int32, [_H, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "arianna_ladder_sums": (C.c_int32, [_H, _D]),
+    "arianna_set_histogram": (C.c_int32, [_H, C.c_int32, C.c_double, C.c_double, C.c_int32, C.c_int32]),
+    "arianna_histogram_accumulate": (C.c_int32, [_H]),
+    "arianna_histogram_read": (C.c_int32, [_H, C.c_void_p, C.c_void_p, C.POINTER(C.c_int64)]),
+    "arianna_histogram_reset": (C.c_int32, [_H]),
     "arianna_set_params": (C.c_int32, [_H, C.c_int32, _D, C.c_int32, _D]),
     "arianna_get_params": (C.c_int32, [_H, C.c_int32, _D, C.c_int32]),
     "arianna_sweep": (C.c_int32, [_H, C.c_int64, C.c_uint32]),

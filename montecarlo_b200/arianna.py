@@ -39,6 +39,7 @@ __all__ = [
     "StoreCallbacks", "StoreTrajectories", "StoreLastFrames", "StoreParameters", "PrintTimeSteps",
     "callback_energy", "callback_acceptance", "mc_sweep", "DAT", "TXT", "shard_bounds",
     "ReplicaExchange", "callback_ladder_energy", "callback_ladder_acceptance", "callback_exchange_acceptance",
+    "StoreHistograms",
 ]
 
 
@@ -75,6 +76,20 @@ def allreduce_sums(local: np.ndarray, device_tensor=None) -> np.ndarray:
     t = torch.from_numpy(np.array(local, dtype=np.float64))
     dist.all_reduce(t, op=dist.ReduceOp.SUM)
     return t.numpy()
+
+
+def allreduce_counts(local: np.ndarray) -> np.ndarray:
+    """Sum an int64 array over all ranks, exactly (integer counts must not pass through binary64)."""
+    local = np.ascontiguousarray(local, dtype=np.int64)
+    dist = _dist()
+    if dist is None or dist.get_world_size() == 1:
+        return local
+    import torch
+    t = torch.from_numpy(local.copy())
+    if dist.get_backend() == "nccl":
+        t = t.cuda()
+    dist.all_reduce(t, op=dist.ReduceOp.SUM)
+    return t.cpu().numpy().reshape(local.shape)
 
 
 def means_from_sums(sums: np.ndarray, n_moves: int):
@@ -586,6 +601,76 @@ class StoreCallbacks(AriannaAlgorithm):
             f.close()
 
 
+class StoreHistograms(AriannaAlgorithm):
+    """StoreHistograms(chains; scheduler, path, observable="x", range=(lo, hi), bins, groups=1): the distribution the
+    chains reach, reduced on the device instead of downloading every position.  Each call adds one sample of every
+    chain's current x (or e = potential(x)) to per-group histograms, chain g (global) in group g % groups (groups = L
+    gives the rungs of a ReplicaExchange ladder).  There is no store_first: it samples exactly at its scheduled times
+    t >= 1.  finalise() sums the accumulators over ranks (counts as int64, exactly), keeps them on the instance (`counts`
+    [groups][bins + 3] = bins, underflow, overflow, nan; `moments` [groups][3] = n, Σv, Σv² over the finite values;
+    `samples`) and rank 0 writes `histogram_<observable>.dat`.  Bin of v: floor((v − lo)·inv_w), inv_w = bins / (hi − lo)
+    in binary64 with the subtraction and the product rounded separately; the edges in the file are nominal."""
+
+    def __init__(self, chains, *, path=None, observable: str = "x", range=None, bins=None, groups: int = 1, **extras):
+        if observable not in ("x", "e"):
+            raise ValueError('StoreHistograms: observable must be "x" or "e"')
+        if range is None or len(range) != 2 or bins is None:
+            raise TypeError("StoreHistograms: range=(lo, hi) and bins are required")
+        self.observable = observable
+        self.lo, self.hi = float(range[0]), float(range[1])
+        self.bins, self.groups = int(bins), int(groups)
+        self.path = os.path.join(path, f"histogram_{observable}.dat")
+        self.counts = self.moments = None
+        self.samples = 0
+        self._write = getattr(chains, "rank", 0) == 0
+        self._set = False
+        if self._write:
+            os.makedirs(path, exist_ok=True)
+
+    def initialise(self, simulation):
+        simulation.chains.engine.set_histogram(self.observable, self.lo, self.hi, self.bins, self.groups)
+        self._set = True
+
+    def make_step(self, simulation):
+        ch = simulation.chains
+        ch.flush()
+        ch.engine.histogram_accumulate()
+
+    def finalise(self, simulation):
+        if not self._set:
+            return
+        counts, moments, samples = simulation.chains.engine.histogram()
+        self.counts = allreduce_counts(counts)
+        self.moments = _allreduce_host(moments.reshape(-1)).reshape(moments.shape)
+        self.samples = int(samples)
+        if self._write:
+            with open(self.path, "w") as f:
+                f.write(self.render())
+
+    def render(self) -> str:
+        lo, hi, n, G = self.lo, self.hi, self.bins, self.groups
+        out = [f"# StoreHistograms: {self.observable}",
+               f"# lo = {_jl(lo)}, hi = {_jl(hi)}, bins = {n}, groups = {G}, samples = {self.samples}",
+               f"# bin k holds the v with floor((v - lo) * inv_w) == k, inv_w = bins / (hi - lo) = {_jl(n / (hi - lo))} "
+               "(binary64, the subtraction and the product rounded separately); left and right are the nominal edges "
+               "lo + k (hi - lo) / bins",
+               "# left right count[group 0] ... count[group groups-1]; then underflow, overflow and nan; then one "
+               "'moments n sum(v) sum(v^2)' line per group, over the finite v"]
+        for k in range(n):
+            left, right = lo + k * (hi - lo) / n, lo + (k + 1) * (hi - lo) / n
+            out.append(f"{_jl(left)} {_jl(right)} " + " ".join(str(int(c)) for c in self.counts[:, k]))
+        for j, name in enumerate(("underflow", "overflow", "nan")):
+            out.append(f"{name} " + " ".join(str(int(c)) for c in self.counts[:, n + j]))
+        for m in self.moments:
+            out.append(f"moments {int(m[0])} {_jl(float(m[1]))} {_jl(float(m[2]))}")
+        return "\n".join(out) + "\n"
+
+    def write_algorithm(self, io, scheduler):
+        io.write(f"\tStoreHistograms\n\t\tCalls: {sum(1 for x in scheduler if 0 < x <= scheduler[-1])}\n")
+        io.write(f"\t\tObservable: {self.observable}\n\t\tRange: {_jl([self.lo, self.hi])}\n")
+        io.write(f"\t\tBins: {self.bins}\n\t\tGroups: {self.groups}\n")
+
+
 class DAT:
     extension = ".dat"
 
@@ -803,7 +888,9 @@ def _make_lookahead(sim: "Simulation"):
     fires at time t the ensemble can run every following store interval up to the next event that observes or
     changes the chains in any other way (trajectory frames, the PGMC estimator/update, parameter stores, ...) as ONE
     arianna_sweep_series call.  Returns a function () -> [K_1, K_2, ...] (MC steps between the coming callback-only
-    store times, as of sim.t), or None when the algorithm list does not allow it."""
+    store times, as of sim.t), or None when the algorithm list does not allow it.  Algorithms this planner does not
+    know -- ReplicaExchange, StoreHistograms, ... -- are neither StoreCallbacks nor passive, so their times are barriers:
+    a stretch stops there, and the callback-only stores between two such times are still fused."""
     import bisect
     algs = sim.algorithms
     met = [k for k, a in enumerate(algs) if isinstance(a, Metropolis)]

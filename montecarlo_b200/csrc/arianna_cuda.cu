@@ -18,6 +18,7 @@
 #include "../../include/arianna_cuda.h"
 #include "kernels.cuh"
 #include "kernels_exchange.cuh"
+#include "kernels_histogram.cuh"
 
 using namespace arianna;
 
@@ -63,6 +64,8 @@ static const char *load(std::string &err)
 static_assert(ARIANNA_MAX_MOVES == kMaxMoves, "header / kernel pool size mismatch");
 static_assert(ARIANNA_MAX_SERIES == kMaxSeries, "header / kernel series size mismatch");
 static_assert(ARIANNA_MAX_LADDER == kMaxLadder, "header / kernel ladder size mismatch");
+static_assert(ARIANNA_MAX_HISTOGRAM_CELLS == kHistMaxCells, "header / kernel histogram size mismatch");
+static_assert(kHistBlock >= kMaxLadder, "every group needs a thread in every CTA of histogram_kernel");
 static_assert(sizeof(arianna_gradient_data) == 5 * sizeof(double), "gradient record layout");
 
 struct arianna_handle {
@@ -138,6 +141,15 @@ struct arianna_handle {
     double *d_ladder = nullptr;            // [L] the β ladder
     double *d_ladder_partials = nullptr;   // [grid][L][1 + n_moves] of ladder_reduce_kernel
     double *d_ladder_sums = nullptr;       // [L][2 + n_moves]
+
+    int hist_obs = -1;                     // on-device histogram: observable (-1 = none set)
+    int hist_bins = 0, hist_groups = 0, hist_grid = 0;
+    size_t hist_smem = 0;                  // dynamic shared memory of histogram_kernel: G·(n_bins + 3) u32
+    double hist_lo = 0.0, hist_inv_w = 0.0;
+    int64_t hist_samples = 0;              // accumulate calls since set / reset
+    unsigned long long *d_hist_counts = nullptr;   // [G][n_bins + 3]
+    double *d_hist_moments = nullptr;      // [G][3]
+    double *d_hist_partials = nullptr;     // [hist_grid][G][3]
     std::string err;
 };
 
@@ -350,6 +362,18 @@ int32_t dispatch_pot(int pot, F &&f)
     }
 }
 
+// f(kernel) with the histogram_kernel instantiation of the handle's element type, the observable and the potential
+template <typename F>
+int32_t dispatch_histogram(const arianna_handle *h, int observable, F &&f)
+{
+    auto pick = [&](auto zero) -> int32_t {
+        using T = decltype(zero);
+        if (observable == ARIANNA_OBS_X) return f(histogram_kernel<T, kHistPosition>);
+        return dispatch_pot(h->cfg.potential, [&](auto pot) -> int32_t { return f(histogram_kernel<T, decltype(pot)::value>); });
+    };
+    return h->f32 ? pick(0.0f) : pick(0.0);
+}
+
 }  // namespace
 
 extern "C" {
@@ -520,6 +544,7 @@ int32_t arianna_destroy(arianna_handle *h)
     cudaFree(h->d_series); cudaFree(h->d_series_partials); cudaFree(h->d_cat_table);
     cudaFree(h->d_pgmc_partials); cudaFree(h->d_pgmc_ticket); cudaFree(h->d_theta);
     cudaFree(h->d_xacc); cudaFree(h->d_ladder); cudaFree(h->d_ladder_partials); cudaFree(h->d_ladder_sums);
+    cudaFree(h->d_hist_counts); cudaFree(h->d_hist_moments); cudaFree(h->d_hist_partials);
     if (h->coll_stream) cudaStreamSynchronize(h->coll_stream);
     if (h->comm) { nccl::g_api.CommDestroy(h->comm); h->comm = nullptr; }
     cudaFree(h->d_coll);
@@ -1612,6 +1637,117 @@ int32_t arianna_ladder_sums(arianna_handle *h, double *sums)
     ++h->launches;
     CU_TRY(h, cudaMemcpyAsync(sums, h->d_ladder_sums, sizeof(double) * L * (2 + nm), cudaMemcpyDeviceToHost, h->stream));
     CU_TRY(h, cudaStreamSynchronize(h->stream));
+    return ARIANNA_OK;
+}
+
+// ---- on-device histograms and moments of x or e (csrc/kernels_histogram.cuh) ---------------------------------------
+static int32_t histogram_set(arianna_handle *h, const char *who)
+{
+    REQUIRE(h, h->hist_obs >= 0, std::string(who) + ": no histogram (call arianna_set_histogram first)");
+    return ARIANNA_OK;
+}
+
+int32_t arianna_set_histogram(arianna_handle *h, int32_t observable, double lo, double hi, int32_t n_bins, int32_t n_groups)
+{
+    if (!h) return ARIANNA_ERR_INVALID;
+    REQUIRE(h, observable == ARIANNA_OBS_X || observable == ARIANNA_OBS_E, "arianna_set_histogram: unknown observable");
+    REQUIRE(h, n_bins >= 1, "arianna_set_histogram: n_bins must be >= 1");
+    REQUIRE(h, n_groups >= 1 && n_groups <= ARIANNA_MAX_LADDER, "arianna_set_histogram: n_groups must be in 1..ARIANNA_MAX_LADDER");
+    REQUIRE(h, (int64_t)n_groups * ((int64_t)n_bins + 3) <= ARIANNA_MAX_HISTOGRAM_CELLS,
+            "arianna_set_histogram: n_groups * (n_bins + 3) exceeds ARIANNA_MAX_HISTOGRAM_CELLS");
+    REQUIRE(h, std::isfinite(lo) && std::isfinite(hi) && lo < hi, "arianna_set_histogram: lo and hi must be finite, lo < hi");
+    const double inv_w = (double)n_bins / (hi - lo);
+    REQUIRE(h, std::isfinite(inv_w) && inv_w > 0.0, "arianna_set_histogram: n_bins / (hi - lo) must be finite and > 0");
+    DeviceGuard guard(h->device);
+    CU_TRY(h, cudaStreamSynchronize(h->stream));   // an accumulate in flight still uses the old buffers
+    cudaFree(h->d_hist_counts); cudaFree(h->d_hist_moments); cudaFree(h->d_hist_partials);
+    h->d_hist_counts = nullptr;
+    h->d_hist_moments = h->d_hist_partials = nullptr;
+    h->hist_obs = -1;
+    const int G = n_groups, cells = n_groups * (n_bins + 3);
+    const size_t smem = sizeof(unsigned int) * cells;
+    int per_sm = 0;
+    int32_t rc = dispatch_histogram(h, observable, [&](auto kernel) -> int32_t {
+        CU_TRY(h, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                       (int)(sizeof(unsigned int) * kHistMaxCells)));
+        CU_TRY(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kHistBlock, smem));
+        return ARIANNA_OK;
+    });
+    if (rc) return rc;
+    if (per_sm < 1) return fail(h, ARIANNA_ERR_CUDA, "arianna_set_histogram: histogram_kernel cannot be resident");
+    // one resident wave: every CTA flushes its whole histogram once, so more CTAs only cost more global atomics
+    const int64_t need = (h->M + kHistBlock - 1) / kHistBlock;
+    const int64_t wave = (int64_t)h->sm_count * per_sm;
+    const int grid = (int)(need < wave ? need : wave);
+    CU_TRY(h, cudaMalloc(&h->d_hist_counts, sizeof(unsigned long long) * cells));
+    CU_TRY(h, cudaMalloc(&h->d_hist_moments, sizeof(double) * G * 3));
+    CU_TRY(h, cudaMalloc(&h->d_hist_partials, sizeof(double) * (size_t)grid * G * 3));
+    CU_TRY(h, cudaMemsetAsync(h->d_hist_counts, 0, sizeof(unsigned long long) * cells, h->stream));
+    CU_TRY(h, cudaMemsetAsync(h->d_hist_moments, 0, sizeof(double) * G * 3, h->stream));
+    h->hist_obs = observable;
+    h->hist_bins = n_bins;
+    h->hist_groups = G;
+    h->hist_grid = grid;
+    h->hist_smem = smem;
+    h->hist_lo = lo;
+    h->hist_inv_w = inv_w;
+    h->hist_samples = 0;
+    return ARIANNA_OK;
+}
+
+int32_t arianna_histogram_accumulate(arianna_handle *h)
+{
+    if (!h) return ARIANNA_ERR_INVALID;
+    if (int32_t rc = histogram_set(h, "arianna_histogram_accumulate")) return rc;
+    DeviceGuard guard(h->device);
+    const int G = h->hist_groups;
+    HistogramParams p{};
+    p.x = h->f32 ? static_cast<const void *>(h->d_xf) : static_cast<const void *>(h->d_x);
+    p.M = h->M;
+    p.g0 = (int)(((h->cfg.chain_offset % G) + G) % G);
+    p.G = G;
+    p.n_bins = h->hist_bins;
+    p.lo = h->hist_lo;
+    p.inv_w = h->hist_inv_w;
+    p.counts = h->d_hist_counts;
+    p.partials = h->d_hist_partials;
+    dispatch_histogram(h, h->hist_obs, [&](auto kernel) -> int32_t {
+        kernel<<<h->hist_grid, kHistBlock, h->hist_smem, h->stream>>>(p);
+        return ARIANNA_OK;
+    });
+    CU_TRY(h, cudaGetLastError());
+    ++h->launches;
+    histogram_fold_kernel<<<G, kBlock, 0, h->stream>>>(h->d_hist_partials, h->hist_grid, G, h->d_hist_moments);
+    CU_TRY(h, cudaGetLastError());
+    ++h->launches;
+    ++h->hist_samples;
+    return ARIANNA_OK;
+}
+
+int32_t arianna_histogram_read(arianna_handle *h, int64_t *counts, double *moments, int64_t *n_samples)
+{
+    if (!h) return ARIANNA_ERR_INVALID;
+    if (int32_t rc = histogram_set(h, "arianna_histogram_read")) return rc;
+    DeviceGuard guard(h->device);
+    const size_t G = (size_t)h->hist_groups;
+    if (counts)
+        CU_TRY(h, cudaMemcpyAsync(counts, h->d_hist_counts, sizeof(int64_t) * G * (h->hist_bins + 3), cudaMemcpyDeviceToHost,
+                                  h->stream));
+    if (moments) CU_TRY(h, cudaMemcpyAsync(moments, h->d_hist_moments, sizeof(double) * G * 3, cudaMemcpyDeviceToHost, h->stream));
+    CU_TRY(h, cudaStreamSynchronize(h->stream));
+    if (n_samples) *n_samples = h->hist_samples;
+    return ARIANNA_OK;
+}
+
+int32_t arianna_histogram_reset(arianna_handle *h)
+{
+    if (!h) return ARIANNA_ERR_INVALID;
+    if (int32_t rc = histogram_set(h, "arianna_histogram_reset")) return rc;
+    DeviceGuard guard(h->device);
+    const size_t G = (size_t)h->hist_groups;
+    CU_TRY(h, cudaMemsetAsync(h->d_hist_counts, 0, sizeof(unsigned long long) * G * (h->hist_bins + 3), h->stream));
+    CU_TRY(h, cudaMemsetAsync(h->d_hist_moments, 0, sizeof(double) * G * 3, h->stream));
+    h->hist_samples = 0;
     return ARIANNA_OK;
 }
 

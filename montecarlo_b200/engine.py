@@ -209,6 +209,35 @@ class CudaEnsemble:
         self._ck(self._lib.arianna_ladder_sums(self._h, out.ctypes.data_as(C.POINTER(C.c_double))))
         return out
 
+    # -- on-device histograms -------------------------------------------------------------------------------
+    def set_histogram(self, observable, lo: float, hi: float, n_bins: int, n_groups: int = 1):
+        """Histogram and moments of observable "x" (position) or "e" (energy) over [lo, hi) in n_bins bins, per group of
+        chains g % n_groups (g global), accumulated on the device (arianna_set_histogram).  Bin of v:
+        floor((v − lo)·inv_w) with inv_w = n_bins / (hi − lo) in binary64, the subtraction and the product rounded
+        separately; NaN, below and above the range go to their own cells."""
+        # an unknown name goes to the library as -1, which refuses it like every other bad argument (ERR_INVALID)
+        obs = L.OBSERVABLES.get(observable, -1) if isinstance(observable, str) else int(observable)
+        self._ck(self._lib.arianna_set_histogram(self._h, int(obs), float(lo), float(hi), int(n_bins), int(n_groups)))
+        self._hist_shape = (int(n_groups), int(n_bins) + 3)
+
+    def histogram_accumulate(self):
+        """Add one sample of every local chain's current state to the accumulators (asynchronous; reads x only)."""
+        self._ck(self._lib.arianna_histogram_accumulate(self._h))
+
+    def histogram(self):
+        """(counts int64 [G][n_bins + 3] = [bins..., underflow, overflow, nan], moments f64 [G][3] = (n, Σv, Σv²) over the
+        finite values, number of accumulate calls) of the local shard."""
+        shape = getattr(self, "_hist_shape", None)
+        counts = np.empty(shape, dtype=np.int64) if shape else None
+        moments = np.empty((shape[0], 3), dtype=np.float64) if shape else None
+        n = C.c_int64()
+        self._ck(self._lib.arianna_histogram_read(self._h, _ptr(counts), _ptr(moments), C.byref(n)))
+        return counts, moments, n.value
+
+    def histogram_reset(self):
+        """Zero counts, moments and the call count; the binning stays."""
+        self._ck(self._lib.arianna_histogram_reset(self._h))
+
     # -- policy parameters --------------------------------------------------------------------------------
     def set_params(self, move_id: int, sigma: float, log_norm: Optional[float] = None):
         th = C.c_double(float(sigma))
